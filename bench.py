@@ -55,7 +55,14 @@ def parse_args():
     ap.add_argument("--index", default="auto", choices=["auto", "replicated", "sharded"],
                     help="prefix index placement at N > 1: sharded = BASELINE config 4 (hash-range shards, index N x "
                          "--index-keys, one NCCL all-to-all each way per batch); auto = sharded when N > 1")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (rank 0's requests, "
+                                                          "a fixed sample of rows) to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the CUDA path's results (--impl b200)")
+    return args
 
 
 def host_threads():
@@ -197,6 +204,41 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_ROWS = 1024
+DUMP_BYTES = 56 << 20
+
+
+def dump_outputs(out_dir, d_ids, d_nids, d_st, d_keys, d_match, d_route):
+    """Writes the results of the device-resident step — what xllm_ingest_batch would hand a caller: token ids, their
+    count and status, block keys, match and routing — as float32 / float64 arrays (exact for every value stored) to
+    out_dir/<name>.npy.  A fixed seeded sample of rows (rows.npy) keeps the files under 64 MB, so two builds run
+    with the same arguments can be compared output for output."""
+    import torch
+    from xllm_service_b200 import _lib
+    n, T = d_ids.shape
+    nb = d_keys.shape[1]
+    row_bytes = 8 * T + 4 * 16 * nb + 4 * 4 * 64 + 8 * 10
+    rows = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_ROWS, DUMP_BYTES // row_bytes), replace=False))
+    idx = torch.from_numpy(rows).to(d_ids.device)
+    take = lambda t: t.index_select(0, idx).cpu().numpy()  # noqa: E731
+    match = take(d_match).view(_lib.MATCH_DTYPE)[:, 0]
+    route = take(d_route).view(_lib.ROUTING_DTYPE)[:, 0]
+    inst = match["instances"][:, None] >> np.arange(64, dtype=np.uint64) & np.uint64(1)
+    out = {"rows": rows.astype(np.float64), "ids": take(d_ids).astype(np.float64),
+           "n_ids": take(d_nids).astype(np.float64), "status": take(d_st).astype(np.float64),
+           "keys": take(d_keys).astype(np.float32),
+           "match_max_block_num": match["max_block_num"].astype(np.float64),
+           "match_max_matched_block_num": match["max_matched_block_num"].astype(np.float64),
+           "match_instances": inst.astype(np.float32)}
+    for f in ("hbm", "dram", "ssd"):
+        out["match_" + f] = match[f].astype(np.float32)
+    for f in ("prefill_id", "decode_id", "ok", "prefill_score", "decode_score"):
+        out["routing_" + f] = route[f].astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def peaks():
@@ -791,6 +833,8 @@ def main():
     k_ms = np.array([[e[i].elapsed_time(e[i + 1]) for i in range(3)] for e in ev]).mean(axis=0)
     assert (torch.equal(d_ids.cpu(), torch.from_numpy(h_ids.numpy())) and
             torch.equal(d_keys.cpu(), torch.from_numpy(h_keys.numpy()))), "device-resident != e2e results"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_ids, d_nids, d_st, d_keys, d_match, d_route)
 
     shard_stats = h.shard_last_stats() if sharded_mode else None   # the last device-resident step's round
 
